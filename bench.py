@@ -2,6 +2,7 @@
 """bench.py -- image-pairs/sec of the UniMatch matching path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config4|config2|config3|config5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -12,6 +13,9 @@ Prints ONE JSON line (rank 0).  `value`: inputs resident in HBM; `e2e`: host pin
 the timed region.  `--impl reference` times the CPU oracle port of the reference path on the host's physical cores.
 `epe_vs_reference` compares pair 0 of the GPU output with the oracle (== reference) and carries its tolerance and a pass flag;
 a failing parity check makes the process exit non-zero after printing the line.
+`--dump-outputs DIR` writes the prediction of the last timed step (rank 0) as DIR/<flow|disparity|depth>.npy, float32, at
+most 64 MB (a larger output is cut to a seeded sample of whole pairs, listed in the JSON line).  Inputs and weights are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -25,6 +29,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "image-pairs/sec @480x832 gmflow-scale2-refine6; EPE vs reference"
 # name -> (workload, H, W, pairs per GPU, BASELINE.json configs index, metric string, (mean tol, max tol, unit))
@@ -115,6 +120,26 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx, "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_LIMIT = 64 * 10 ** 6               # bytes written by --dump-outputs
+
+
+def dump_outputs(directory, task, out):
+    """Write `out` ([B,2,H,W] flow or [B,H,W] disparity / depth) as float32 .npy under `directory`; above DUMP_LIMIT a
+    seeded sample of whole pairs is written instead.  Returns what was written, for the JSON line."""
+    import numpy as np
+    name = {"flow": "flow", "stereo": "disparity", "depth": "depth"}[task] + ".npy"
+    out = out.detach().float().cpu()
+    pairs = None
+    if out.numel() * 4 > DUMP_LIMIT:
+        k = DUMP_LIMIT // (out[0].numel() * 4)
+        pairs = torch.randperm(out.shape[0], generator=torch.Generator().manual_seed(0))[:k].sort().values
+        out = out[pairs]
+        pairs = pairs.tolist()
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name), out.numpy())
+    return {"dir": os.path.abspath(directory), "files": {name: list(out.shape)}, "pairs": pairs}
+
+
 def run_oracle_once(sd, cfg, batch, threads, device="cpu"):
     """One forward of the oracle port (the reference's own ATen op sequence, oracle/unimatch_oracle.py)."""
     from oracle import unimatch_oracle as O
@@ -148,6 +173,7 @@ def main():
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip the reference-eager-on-this-GPU line (oracle port on cuda, TF32 off)")
     ap.add_argument("--profile", action="store_true", help="1 warm-up + K steps of the resident path only (for ncu launch lists)")
     ap.add_argument("--graph", action="store_true", help="replay the forward as a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's prediction as DIR/<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -178,13 +204,14 @@ def main():
         t_start = time.perf_counter()
         times = []
         for i in range(args.warmup + args.steps):
-            _, dt = run_oracle_once(sd, cfg, batch, ncores)
+            out, dt = run_oracle_once(sd, cfg, batch, ncores)
             if i >= args.warmup or (time.perf_counter() - t_start) > budget:
                 times.append(dt)
             if (time.perf_counter() - t_start) > budget and times:
                 break
         sec = sum(times) / len(times)
         val = 1.0 / sec
+        dumped = {"dump_outputs": dump_outputs(args.dump_outputs, task, out)} if args.dump_outputs else {}
         print(json.dumps({
             "impl": "reference", "metric": metric, "value": val, "unit": "pairs/s", "n_gpus": args.gpus,
             "steps": len(times), "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": sec * 1e3,
@@ -192,7 +219,7 @@ def main():
             "config": config,
             "cpu_baseline": {"value": val, "unit": "pairs/s", "cores": ncores, "host_logical_cpus": os.cpu_count(), "kind": "port",
                              "sample": "1 pair per step, %d timed steps (240 s budget), torch threads = physical cores" % len(times)},
-            "e2e": {"value": val, "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
+            "e2e": {"value": val, "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, **dumped}))
         return
 
     # ------------------------------------------------------------------ our arm
@@ -266,9 +293,12 @@ def main():
                 pending[i].wait()
                 pending[i] = None
 
+    last = [None]                                          # the prediction of the latest resident step
+
     def step_resident():
         flow = forward()
         gather_async(flow)
+        last[0] = flow
         return flow
 
     # End-to-end path: every step's inputs come from pinned host memory and its result goes back to pinned host memory,
@@ -360,12 +390,15 @@ def main():
     if args.profile:
         step_resident()
         ms, launches, _, _ = timed(step_resident, args.steps)
-        print(json.dumps({"profile_run": True, "ms_per_step": ms / args.steps, "gpu_launches": launches}))
+        dumped = {"dump_outputs": dump_outputs(args.dump_outputs, task, last[0])} if args.dump_outputs and rank == 0 else {}
+        print(json.dumps({"profile_run": True, "ms_per_step": ms / args.steps, "gpu_launches": launches, **dumped}))
         return
     for _ in range(max(args.warmup, 3)):
         step_resident()
     gather_drain()
     ms, launches_r, clocks, (ms_own, steps_ms) = timed(step_resident, args.steps, sample_clocks=True, per_step=True)
+    # copied now: with --graph the later passes replay into the same output buffer
+    dumped = dump_outputs(args.dump_outputs, task, last[0]) if args.dump_outputs and rank == 0 else None
     # kernel-level timers and the launch counter live in the eager path: a separate pass (events around every launch group
     # perturb the host side, so this pass is not the one `value` is taken from)
     timer = {}
@@ -455,6 +488,8 @@ def main():
               "roofline": roofline, "roofline_conv": roofline_conv, "roofline_attention_simt": roofline_simt,
               "sections_ms_per_step": {k[4:]: round(v[0] / args.steps, 3) for k, v in timer.items() if k.startswith("sec:")},
               "ranks": rank_stats, "gather_only_ms": gather_ms}
+    if dumped:
+        result["dump_outputs"] = dumped
 
     parity_ok = True
     if rank == 0 and world == 1 and not args.no_cpu_baseline:

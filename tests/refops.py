@@ -352,3 +352,9 @@ def register_cpu_kernels():
     for name in ALL:
         lib.impl(name, g[name])
     _registered.append(lib)
+
+
+def unregister_cpu_kernels():
+    """Remove the CPU kernels installed by `register_cpu_kernels()`: the ops are back to the product's, which have none."""
+    while _registered:
+        _registered.pop()._destroy()

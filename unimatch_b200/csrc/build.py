@@ -40,7 +40,7 @@ if os.environ.get("UM_ATTN_DEBUG_BUILD") == "1":      # diagnostics of the atten
 
 def _stamp():
     h = hashlib.sha256()
-    h.update(" ".join(FLAGS).encode())
+    h.update(" ".join(FLAGS).replace(ROOT, "").encode())       # a moved checkout keeps its library
     for f in sorted(os.listdir(HERE)) + [os.path.join(ROOT, "include", "unimatch_sm100.h")]:
         p = f if os.path.isabs(f) else os.path.join(HERE, f)
         if p.endswith((".cu", ".cuh", ".h", "build.py")):
