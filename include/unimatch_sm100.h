@@ -124,6 +124,15 @@ int um_local_corr_softmax(const float* f0, const float* f1, float* flow,
  * Replaces local_correlation_with_flow (matching.py:86-123). */
 int um_local_corr_volume(const float* f0, const float* f1, const float* flow, float* corr,
                          int32_t batch, int32_t h, int32_t w, int32_t radius, int32_t flow_dim, void* stream);
+/* The same volume from fp16 (hi, lo) feature planes f0_planes / f1_planes [2][B][h][w][128] (um_split_planes), on the
+ * tcgen05 tensor cores: one GEMM per 16 x 8 pixel tile against f1 over the bounding box of the tile's windows, with
+ * fp32-faithful 3xFP16 dot products.  Tiles whose box is too large (a rough flow) are computed on CUDA cores instead;
+ * fallback_tiles (device int32 or NULL) receives their number.  Outputs: corr (fp32 [B,h,w,81], or NULL) and/or out_split
+ * (fp16 (hi, lo) planes [2][B][h][w][cp_split], channels [off_split, off_split + 81) written, the others untouched; or
+ * NULL), the split being that of um_split_planes. */
+int um_local_corr_volume_planes(const void* f0_planes, const void* f1_planes, const float* flow, float* corr,
+                                void* out_split, int32_t cp_split, int32_t off_split, int32_t batch, int32_t h, int32_t w,
+                                int32_t radius, int32_t flow_dim, int32_t* fallback_tiles, void* stream);
 
 /* out[b,y,x,:] = bilinear(f[b], x + u, y + v), zeros outside, align_corners=True; (u,v) as above.
  * Replaces flow_warp (geometry.py:65-72, bilinear_sample :41-62). */

@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 LIB = os.path.join(os.path.dirname(HERE), "libunimatch_sm100.so")
-SOURCES = ["um_api.cu", "um_attention_simt.cu", "um_attention_tc.cu", "um_attention_tc2.cu", "um_conv_tc.cu", "um_ffn_tc.cu", "um_local.cu", "um_local_stencil.cu", "um_misc.cu", "um_norm.cu", "um_stem.cu"]
+SOURCES = ["um_api.cu", "um_attention_simt.cu", "um_attention_tc.cu", "um_attention_tc2.cu", "um_conv_tc.cu", "um_ffn_tc.cu", "um_local.cu", "um_local_tc.cu", "um_local_stencil.cu", "um_misc.cu", "um_norm.cu", "um_stem.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "-I", os.path.join(ROOT, "include"), "-I", HERE]
 

@@ -12,42 +12,14 @@
 #include <math_constants.h>
 
 #include "um_common.cuh"
+#include "um_local_tap.cuh"
 
 namespace {
 
-constexpr float SQRT_C = 11.313708498984761f;
+using namespace um::local;
+
 constexpr int PIX_PER_CTA = 32;     // 256 threads = 8 warps x 4 pixels
 
-struct Tap { int x0, y0; float wnw, wne, wsw, wse; };
-
-__device__ __forceinline__ float unnormalize(float g, int size) { return ((g + 1.0f) / 2.0f) * (float)(size - 1); }
-
-// geometry.py:49-51 normalisation (bilinear_sample): g = 2*p/(size-1) - 1
-__device__ __forceinline__ float norm_sample(float p, int size) { return 2.0f * p / (float)(size - 1) - 1.0f; }
-// geometry.py:35-38 normalisation (normalize_coords): g = (p - c)/c, c = (size-1)/2
-__device__ __forceinline__ float norm_window(float p, int size) { float c = (float)(size - 1) / 2.0f; return (p - c) / c; }
-
-__device__ __forceinline__ Tap make_tap(float ix, float iy) {
-  Tap t;
-  float fx = floorf(ix), fy = floorf(iy);
-  t.x0 = (int)fx; t.y0 = (int)fy;
-  float xe = fx + 1.0f, ye = fy + 1.0f;
-  t.wnw = (xe - ix) * (ye - iy);
-  t.wne = (ix - fx) * (ye - iy);
-  t.wsw = (xe - ix) * (iy - fy);
-  t.wse = (ix - fx) * (iy - fy);
-  return t;
-}
-
-struct Vec16 { float4 v[4]; };
-
-__device__ __forceinline__ Vec16 load_row(const float* row, int sub) {
-  Vec16 r;
-  const float4* p = reinterpret_cast<const float4*>(row);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) r.v[i] = __ldg(p + sub + 8 * i);
-  return r;
-}
 __device__ __forceinline__ void store_row(float* row, int sub, const Vec16& r) {
   float4* p = reinterpret_cast<float4*>(row);
 #pragma unroll
@@ -66,25 +38,6 @@ __device__ __forceinline__ void axpy(Vec16& acc, float w, const Vec16& x) {
     acc.v[i].z = fmaf(w, x.v[i].z, acc.v[i].z); acc.v[i].w = fmaf(w, x.v[i].w, acc.v[i].w);
   }
 }
-__device__ __forceinline__ float dot_partial(const Vec16& a, const Vec16& b) {
-  float s = 0.f;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    s = fmaf(a.v[i].x, b.v[i].x, s); s = fmaf(a.v[i].y, b.v[i].y, s);
-    s = fmaf(a.v[i].z, b.v[i].z, s); s = fmaf(a.v[i].w, b.v[i].w, s);
-  }
-  return s;
-}
-// sum over the 8 lanes of one pixel group; only that group's lanes are named in the mask, so groups whose
-// pixel is out of range may have exited
-__device__ __forceinline__ float reduce8(float s) {
-  const unsigned gmask = 0xFFu << (threadIdx.x & 24);
-  s += __shfl_xor_sync(gmask, s, 4);
-  s += __shfl_xor_sync(gmask, s, 2);
-  s += __shfl_xor_sync(gmask, s, 1);
-  return s;
-}
-
 // bilinear sample of a 128-channel row (zeros padding), ATen order nw, ne, sw, se.  A tap whose weight is exactly zero
 // is not fetched: w * x with w == 0 adds +-0 to a finite accumulator, so the result is bit-identical -- and the integer
 // windows of local_correlation_softmax (matching.py:58-67) land exactly on pixel centres almost everywhere, which makes
@@ -98,11 +51,6 @@ __device__ __forceinline__ Vec16 sample(const float* img, int h, int w, const Ta
   if (yb && xl && t.wsw != 0.0f) axpy(acc, t.wsw, load_row(img + ((long long)(t.y0 + 1) * w + t.x0) * UM_C, sub));
   if (yb && xr && t.wse != 0.0f) axpy(acc, t.wse, load_row(img + ((long long)(t.y0 + 1) * w + t.x0 + 1) * UM_C, sub));
   return acc;
-}
-
-__device__ __forceinline__ void read_flow(const float* flow, long long pix, int flow_dim, float* u, float* v) {
-  if (flow_dim == 2) { float2 f = __ldg(reinterpret_cast<const float2*>(flow) + pix); *u = f.x; *v = f.y; }
-  else { *u = -__ldg(flow + pix); *v = 0.0f; }     // disparity -> (-d, 0)  (unimatch.py:160-166, :277-287)
 }
 
 // ---------------------------------------------------------------------------------------------------------

@@ -17,7 +17,7 @@ LIB_PATH = os.path.join(_HERE, "libunimatch_sm100.so")
 SYMBOLS = [
     "um_abi_version", "um_build_info", "um_last_error", "um_launch_count",
     "um_window_attention", "um_window_attention_workspace", "um_attention_planes_lp", "um_window_attention_planes", "um_debug_set_dump", "um_softmax_expectation", "um_softmax_expectation_workspace",
-    "um_local_corr_softmax", "um_local_corr_volume", "um_flow_warp", "um_fb_consistency", "um_propagate_local", "um_depth_corr_softmax",
+    "um_local_corr_softmax", "um_local_corr_volume", "um_local_corr_volume_planes", "um_flow_warp", "um_fb_consistency", "um_propagate_local", "um_depth_corr_softmax",
     "um_conv2d_tc", "um_ffn_tc", "um_conv7x7_small", "um_split_planes", "um_instance_norm_scratch_floats", "um_instance_norm_stats", "um_instance_norm_apply", "um_add_position", "um_layernorm_residual", "um_convex_upsample", "um_upsample2x", "um_resize_bilinear", "um_gru_rh", "um_gru_update",
 ]
 
@@ -89,6 +89,7 @@ def _load():
         "um_softmax_expectation": [P, P, P, P, I, I, I, L, L, I, I, I, G, P, L, I, P],
         "um_local_corr_softmax": [P, P, P, I, I, I, I, I, I, P],
         "um_local_corr_volume": [P, P, P, P, I, I, I, I, I, P],
+        "um_local_corr_volume_planes": [P, P, P, P, P, I, I, I, I, I, I, I, P, P],
         "um_flow_warp": [P, P, P, I, I, I, I, P],
         "um_fb_consistency": [P, P, F, F, P, P, I, I, I, P],
         "um_propagate_local": [P, P, P, P, I, I, I, I, I, L, L, P],
@@ -293,6 +294,39 @@ def _local_corr_volume(f0, f1, flow, h, w, radius):
 
 local_corr_volume = _define("local_corr_volume(Tensor f0, Tensor f1, Tensor flow, int h, int w, int radius) -> Tensor",
                             _local_corr_volume)
+
+
+def _local_corr_volume_planes(f0_planes, f1_planes, flow, h, w, radius, out_f32, out_split, off_split, fallback_tiles):
+    """local_corr_volume on fp16 (hi, lo) feature planes [2, B, h, w, 128] (tensor cores).  Writes out_f32 [B, h, w, 81]
+    and/or channels [off_split, off_split + 81) of the planes out_split [2, B, h, w, cp]; fallback_tiles (int32 [1]) receives
+    the number of pixel tiles whose flow was too rough for the tensor-core path."""
+    b = f0_planes.shape[1]
+    for t, name in ((f0_planes, "f0_planes"), (f1_planes, "f1_planes")):
+        if t.dtype != torch.float16 or not t.is_contiguous() or tuple(t.shape) != (2, b, h, w, 128):
+            raise RuntimeError("local_corr_volume_planes: %s must be contiguous fp16 planes [2, B, h, w, 128]" % name)
+    _f32c(flow, "flow")
+    if tuple(flow.shape[:3]) != (b, h, w):
+        raise RuntimeError("local_corr_volume_planes: flow must be [B, h, w, 1 or 2]")
+    k = (2 * radius + 1) ** 2
+    if out_f32 is not None:
+        _f32c(out_f32, "out_f32")
+        if tuple(out_f32.shape) != (b, h, w, k):
+            raise RuntimeError("local_corr_volume_planes: out_f32 must be [B, h, w, %d]" % k)
+    cp = 0
+    if out_split is not None:
+        if out_split.dtype != torch.float16 or not out_split.is_contiguous() or tuple(out_split.shape[:4]) != (2, b, h, w):
+            raise RuntimeError("local_corr_volume_planes: out_split must be contiguous fp16 planes [2, B, h, w, cp]")
+        cp = out_split.shape[-1]
+    if fallback_tiles is not None and (fallback_tiles.dtype != torch.int32 or fallback_tiles.numel() < 1):
+        raise RuntimeError("local_corr_volume_planes: fallback_tiles must be an int32 tensor")
+    _check(LIB.um_local_corr_volume_planes(_p(f0_planes), _p(f1_planes), _p(flow), _p(out_f32), _p(out_split), cp, off_split,
+                                           b, h, w, radius, flow.shape[-1], _p(fallback_tiles), _stream()),
+           "um_local_corr_volume_planes")
+
+
+local_corr_volume_planes = _define(
+    "local_corr_volume_planes(Tensor f0_planes, Tensor f1_planes, Tensor flow, int h, int w, int radius, Tensor(a!)? out_f32, "
+    "Tensor(b!)? out_split, int off_split, Tensor(c!)? fallback_tiles) -> ()", _local_corr_volume_planes)
 
 
 def _flow_warp(f, flow, h, w):

@@ -35,6 +35,7 @@ _OPS = torch.ops.unimatch_sm100
 
 import os as _os
 _FUSED_FFN = _os.environ.get("UM_FUSED_FFN", "1") != "0"      # A/B switch of the fused FFN kernel (tools / profiling)
+_CORR_TC = _os.environ.get("UM_CORR_TC", "1") != "0"          # A/B switch of the tensor-core correlation volume (tools / profiling)
 
 
 def _bn256(b, h, w):
@@ -555,14 +556,16 @@ class UniMatch(nn.Module):
 
     def _update_block(self, P, st, corr, flow, want_mask):
         """BasicUpdateBlock.forward (reg_refine.py:106-119) as 11 tensor-core convolutions: activations live as fp16 (hi, lo)
-        planes, the concatenations are channel offsets / second sources, the GRU gate math is the conv epilogue."""
+        planes, the concatenations are channel offsets / second sources, the GRU gate math is the conv epilogue.
+        corr: fp32 correlation volume, or None when it is already in st.corr_s."""
         T, w = P["tc"], P["raw"]
         fd = T["fd"]
         C, L, R = self._conv, ops.CONV_LINEAR, ops.ACT_RELU
-        b, h, wd, _ = corr.shape
-        dev = corr.device
+        b, h, wd, _ = flow.shape
+        dev = flow.device
         bn_zr = bn_fh = _bn256(b, h, wd)
-        _OPS.split_planes(corr, st.corr_s, 0)
+        if corr is not None:
+            _OPS.split_planes(corr, st.corr_s, 0)
         C(st.corr_s, None, *T["convc1"], 1, 1, 0, 0, 256, 256, L, R, None, 0, st.cor1_s, 0, None, None)
         C(st.cor1_s, None, *T["convc2"], 3, 3, 1, 1, 192, 96 if bn_zr == 128 else 192, L, R, None, 0, st.cf_s, 0, None, None)
         _OPS.conv7x7_small(flow, None, False, w["refine.encoder.convf1.weight"], w["refine.encoder.convf1.bias"], 1, True,
@@ -588,6 +591,19 @@ class UniMatch(nn.Module):
             C(st.fh_s, None, *T["mask2"], 1, 1, 0, 0, nm, 64, L, ops.ACT_NONE, mask, 0, None, 0, None, None)
         return st.h2, mask, delta
 
+    @staticmethod
+    def _refine_feature_planes(rst, g0, g1):
+        """fp16 (hi, lo) planes of the correlation features, split once per forward: every iteration reuses them."""
+        cached = getattr(rst, "g_planes", None)
+        if cached is None or cached[0] is not g0 or cached[1] is not g1:
+            planes = []
+            for g in (g0, g1):
+                gs = torch.empty((2,) + tuple(g.shape), device=g.device, dtype=torch.float16)
+                _OPS.split_planes(g, gs, 0)
+                planes.append(gs)
+            rst.g_planes = (g0, g1, planes[0], planes[1])
+        return rst.g_planes[2], rst.g_planes[3]
+
     def _stage_refine_iter(self, P, rst, g0, g1, flow, task, want_mask, depth=None):
         """One regression-refinement iteration (unimatch.py:272-354): 9x9 correlation volume at the current estimate on the
         pre-transformer features, update block, residual update.  Returns (flow, mask or None)."""
@@ -598,7 +614,14 @@ class UniMatch(nn.Module):
         else:
             cflow = flow.contiguous()                                       # disparity handled in-kernel
         with self._section("refine_corr_volume"):
-            corr = _OPS.local_corr_volume(g0, g1, cflow, h, wd, 4)
+            if _CORR_TC and g0.is_cuda:
+                # the volume goes straight into the update block's operand planes (81 of 128 channels).  The op has only a
+                # CUDA kernel (TMA + TMEM); CPU tensors, which only the host-logic tests' oracle kernels accept, keep the fp32 op
+                g0_s, g1_s = self._refine_feature_planes(rst, g0, g1)
+                _OPS.local_corr_volume_planes(g0_s, g1_s, cflow, h, wd, 4, None, rst.corr_s, 0, None)
+                corr = None
+            else:
+                corr = _OPS.local_corr_volume(g0, g1, cflow, h, wd, 4)
         with self._section("refine_update_block"):
             _, mask, delta = self._update_block(P, rst, corr, flow.contiguous(), want_mask)
         if task == "depth":
